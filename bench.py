@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # our arm
     python bench.py --impl reference --gpus N --steps K ...  # CPU restatement of the reference path
     torchrun --nproc-per-node N bench.py --gpus N ...         # one rank per GPU (N>1)
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's outputs as DIR/*.npy
 
 Workload (config.workload "C2", BASELINE.json configs[1]): 2^20 subscribers per GPU all subscribed to
 one topic, batches of 8 broadcast messages with 1 KiB payloads (L=1080 B capnp frame, F=1084 B framed
@@ -27,6 +28,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark may run from a read-only tree and writes nothing into it
 
 METRIC = "broadcast fan-out egress GB/s (1 KiB x 2^20 subscribers per GPU, 1 topic); msgs/s and % of HBM peak alongside"
 N_CONNS = 1 << 20
@@ -51,6 +53,54 @@ def broadcast_frame(topic: int, payload: bytes) -> bytes:
     out += bytes([topic]) + bytes(7)
     out += payload + bytes((-k) % 8)
     return bytes(out)
+
+
+DUMP_SPANS = 1024           # --dump-outputs: spans sampled from the batch's span table
+DUMP_RECORD_BYTES = 12 << 20  # ... and at most this many framed bytes of theirs (48 MB as float32)
+
+
+def dump_outputs(eng, b, out_dir):
+    """--dump-outputs: what a caller of the timed path receives for batch `b` (polled here, released by
+    the caller afterwards), as .npy files that two builds can be compared by:
+      batch.npy    float64 [n_msgs, n_spans, n_deliveries, bytes_out, n_overflow, n_direct_dropped, status]
+      spans.npy    float64 (K, 4): conn, ring_off, len, n_records of a fixed seeded sample of the span
+                   table (sorted by connection, then offset)
+      records.npy  float32: the framed records (4-byte BE length + frame) of those spans, in that order;
+                   the pad bytes up to the 32-byte record stride are unspecified and left out"""
+    import numpy as np
+
+    res = eng.poll(b)
+    if res.runs:   # run-length table {conn0, n_conns, ring_off, len, n_records, off_stride}, expanded without a Python loop
+        r = np.ctypeslib.as_array(C.cast(res.runs, C.POINTER(C.c_uint32)), shape=(res.n_runs, 6)).astype(np.int64)
+        n = r[:, 1]
+        k = np.arange(int(n.sum())) - np.repeat(np.cumsum(n) - n, n)
+        t = np.stack([np.repeat(r[:, 0], n) + k, np.repeat(r[:, 2], n) + k * np.repeat(r[:, 5], n),
+                      np.repeat(r[:, 3], n), np.repeat(r[:, 4], n)], axis=1)
+    elif res.n_spans:
+        t = np.ctypeslib.as_array(C.cast(res.spans, C.POINTER(C.c_uint32)), shape=(res.n_spans, 4)).astype(np.int64)
+    else:
+        t = np.zeros((0, 4), dtype=np.int64)
+    t = t[np.lexsort((t[:, 1], t[:, 0]))]
+    pick = np.sort(np.random.default_rng(0).choice(len(t), size=min(len(t), DUMP_SPANS), replace=False))
+    spans, records, total = [], [], 0
+    for conn, off, ln, nrec in t[pick].tolist():
+        data = eng.read(conn, res.pool_base + off, ln)   # output pool: absolute 32-byte unit offset
+        p, framed = 0, []
+        for _ in range(nrec):
+            n_rec = 4 + int.from_bytes(data[p:p + 4], "big")
+            framed.append(data[p:p + n_rec])
+            p += (n_rec + 31) // 32 * 32
+        framed = b"".join(framed)
+        if total + len(framed) > DUMP_RECORD_BYTES:
+            break
+        spans.append((conn, off, ln, nrec))
+        records.append(framed)
+        total += len(framed)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "batch.npy"), np.array(
+        [res.n_msgs, res.n_spans, res.n_deliveries, res.bytes_out, res.n_overflow, res.n_direct_dropped, res.status], dtype=np.float64))
+    np.save(os.path.join(out_dir, "spans.npy"), np.array(spans, dtype=np.float64).reshape(-1, 4))
+    np.save(os.path.join(out_dir, "records.npy"), np.frombuffer(b"".join(records), dtype=np.uint8).astype(np.float32))
 
 
 def measured_peak():
@@ -199,7 +249,12 @@ def main():
                          "copies the batch from its process's pinned staging (host-buffer path only)")
     ap.add_argument("--host-rings", action="store_true",
                     help="egress hand-off mode: rings in mapped pinned host memory (PCDN_FLAG_HOST_RINGS); PCIe-bound, use with --conns <= 65536")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (batch counters, a seeded sample of its span table and "
+                         "framed records) as DIR/*.npy; with N>1, rank 0's shard")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -298,13 +353,14 @@ def main():
     db.hints = pkg.BATCH_READY
     state = {"i": 0}
 
-    def step_device():
+    def step_device(release=True):
         # the engine double-buffers nothing of the CALLER's: two ingest buffers alternate so that the
         # broadcast of step i+1 (library, ingest stream) never touches the frames step i's pack reads
         k = state["i"] & 1
         state["i"] += 1
         b = eng.submit_device(dbs[k])
-        eng.release_batch(b)                     # the consumer (NIC hand-off) frees the ring space
+        if release:
+            eng.release_batch(b)                 # the consumer (NIC hand-off) frees the ring space
         return b
 
     def drain_device():
@@ -325,11 +381,17 @@ def main():
         launches0 = eng.stats().kernel_launches
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record(stream)
-        for _ in range(args.steps):
-            step_device()
+        for i in range(args.steps):
+            # --dump-outputs: the last batch stays unreleased until its result has been read below (its
+            # release, one small kernel, then runs after the timed window instead of inside it)
+            last = step_device(release=not (args.dump_outputs and i == args.steps - 1))
         drain_device()                        # waits (on the stream) for the last pack
         ev1.record(stream)
         sync_all()
+        if args.dump_outputs:
+            if rank == 0:
+                dump_outputs(eng, last, args.dump_outputs)
+            eng.release_batch(last)
         gpu_launches = int(eng.stats().kernel_launches - launches0)   # counted by the library at every launch site
     ms = ev0.elapsed_time(ev1)
     t_ms = torch.tensor([ms], dtype=torch.float64, device=dev)
@@ -563,7 +625,7 @@ def main():
         secondary = {}
         for wl, extra in (("C4", []), ("C5sparse", []), ("C3", [])):
             try:
-                out = subprocess.run([sys.executable, os.path.join(ROOT, "bench_configs.py"), "--workload", wl, "--steps", "10", "--warmup", "3"] + extra,
+                out = subprocess.run([sys.executable, "-B", os.path.join(ROOT, "bench_configs.py"), "--workload", wl, "--steps", "10", "--warmup", "3"] + extra,
                                      capture_output=True, text=True, timeout=420, check=True)
                 d = json.loads(out.stdout.strip().splitlines()[-1])
                 secondary[wl] = {"workload": d["config"]["workload"], "value": d["value"], "unit": d["unit"], "ms_per_step": d["ms_per_step"],
